@@ -379,6 +379,16 @@ def run_reference_arm(args):
     print(json.dumps(line))
 
 
+def dump_scan_outputs(out_dir, hits, n_hits):
+    """What a caller of the scan job receives: per query the hit count and the (target id, score) list.  Slots past a query's
+    hit count are set to -1, so that equal results give equal files."""
+    valid = np.arange(hits.shape[1])[None, :] < n_hits[:, None].astype(np.int64)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scan_n_hits.npy"), n_hits.astype(np.float64))
+    np.save(os.path.join(out_dir, "scan_hit_ids.npy"), np.where(valid, hits["id"], -1).astype(np.float64))
+    np.save(os.path.join(out_dir, "scan_hit_scores.npy"), np.where(valid, hits["score"], -1).astype(np.float32))
+
+
 def scan_config(args, db_residues, world):
     return {"workload": "ungapped prefilter (BASELINE config[1]): L~350 protein queries vs %d-seq synthetic DB "
                         "(log-normal lengths, %d residues), BLOSUM62 + composition bias; a step = %d queries x the whole DB "
@@ -406,8 +416,12 @@ def main():
     ap.add_argument("--nucl-reads", type=int, default=200000)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=20.0, help="seconds of CPU work for the scan's cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the hit lists of the last timed step (rank 0's queries) to DIR/*.npy, to compare two builds")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and at least one timed step")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -497,6 +511,8 @@ def main():
     launches = ctx.launches - launches0
     clocks = sampler.stop() if rank == 0 else {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
     step_ms = (t_wall * 1e3 if dist is not None else dev_ms)
+    if args.dump_outputs and rank == 0:
+        dump_scan_outputs(args.dump_outputs, *pipe_jobs[(args.steps - 1) % npj].fetch()[:2])
     # kernel-only time of the scan kernel for the roofline (events around the launches of one job, no fetch)
     ctx.event_record(2)
     jobs[0].run()

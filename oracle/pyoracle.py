@@ -187,6 +187,30 @@ class Ref:
     def evalue(self, go, ge, db_residues, score, qlen):
         return float(self.lib.ref_evalue(go, ge, ctypes.c_int64(db_residues), ctypes.c_double(score), ctypes.c_double(qlen), None))
 
+    def evalue_bits(self, go, ge, db_residues, score, qlen):
+        """-> (E-value, bit score) of the gapped statistics"""
+        b = ctypes.c_double(0)
+        e = self.lib.ref_evalue(go, ge, ctypes.c_int64(db_residues), ctypes.c_double(score), ctypes.c_double(qlen), ctypes.byref(b))
+        return float(e), float(b.value)
+
+    def evalue_bits_ungapped(self, db_residues, score, qlen):
+        """-> (E-value, bit score) of the ungapped statistics rescorediagonal uses (EvalueComputation(dbResCount, subMat))"""
+        self.lib.ref_evalue_ungapped.restype = ctypes.c_double
+        b = ctypes.c_double(0)
+        e = self.lib.ref_evalue_ungapped(ctypes.c_int64(db_residues), ctypes.c_double(score), ctypes.c_double(qlen), ctypes.byref(b))
+        return float(e), float(b.value)
+
+    def tantan_matrix(self):
+        lr = np.zeros((21, 21), np.float64)
+        self.lib.ref_tantan_matrix(_p(lr))
+        return lr
+
+    def tantan_probabilities(self, seq):
+        s = np.ascontiguousarray(seq, np.uint8)
+        out = np.zeros(len(s), np.float32)
+        self.lib.ref_tantan_probabilities(_p(s), len(s), _p(out))
+        return out
+
     # ---- `align` module at record level (ref_glue.cpp: ref_align_query) ----
     def align_query(self, q, qkey, tdata, toff, hit_idx, hit_keys, db_residues, comp_bias=True, comp_bias_scale=1.0, go=11, ge=1,
                     sw_mode=2, eval_thr=1e-3, cov_thr=0.0, cov_mode=0, seq_id_thr=0.0, aln_len_thr=0, seq_id_mode=0,

@@ -58,13 +58,9 @@ def test_reader_on_reference_files(gold, tmp_path):
         db.DB(str(tmp_path / "missing"))
 
 
-def test_reader_writer_against_live_reference(tmp_path):
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref not built here")
-    ref = Ref()
+def test_reader_writer_against_live_reference(tmp_path, ref):
     rng = np.random.default_rng(8)
-    keys = rng.permutation(5000)[:400].astype(np.uint32)
+    keys = rng.permutation(5000)[:100].astype(np.uint32)
     ents = [bytes(rng.integers(32, 127, int(rng.integers(0, 300))).astype(np.uint8)) + b"\n" for _ in keys]
     ref.db_write(str(tmp_path / "r"), 0, keys, ents)
     db.write_db(str(tmp_path / "m"), 0, keys, ents)
@@ -111,13 +107,9 @@ def test_reader_on_reference_compressed_files(tmp_path):
         db.DB(bad)
 
 
-def test_compressed_reader_against_live_reference(tmp_path):
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref not built here")
-    ref = Ref()
+def test_compressed_reader_against_live_reference(tmp_path, ref):
     rng = np.random.default_rng(9)
-    keys = rng.permutation(5000)[:300].astype(np.uint32)
+    keys = rng.permutation(5000)[:50].astype(np.uint32)
     aa = np.frombuffer(b"ACDEFGHIKLMNPQRSTVWY", np.uint8)
     ents = [bytes(aa[rng.integers(0, 20, int(rng.integers(0, 900)))]) + b"\n" for _ in keys]
     ref.db_write(str(tmp_path / "c"), 0, keys, ents, compressed=True)

@@ -1,11 +1,11 @@
-"""A7, nucleotide gapped aligner.  CPU: oracle/oracle_ksw.c against the reference fixture (tests/golden/nucl_v1.npz) and,
-where oracle/_ref exists, against the reference's own ksw_extz2_sse / BandedNucleotideAligner on fresh random inputs.
+"""A7, nucleotide gapped aligner.  CPU: oracle/oracle_ksw.c against the reference fixture (tests/golden/nucl_v1.npz) and against
+the reference's own ksw_extz2_sse / BandedNucleotideAligner on seeded random inputs (the `ref` fixture).
 GPU (-m gpu): b200_nucl_align against the fixture and the oracle."""
 import numpy as np
 import pytest
 
 from mmseqs2_b200 import synth
-from oracle.pyoracle import KswOracle, Ref
+from oracle.pyoracle import KswOracle
 
 
 @pytest.fixture(scope="module")
@@ -37,12 +37,10 @@ def test_oracle_matches_reference_fixture(nucl, kso):
     assert gaps > 100
 
 
-@pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built")
-def test_ksw_restatement_vs_reference_random(kso):
-    ref = Ref()
+def test_ksw_restatement_vs_reference_random(kso, ref):
     nmat = kso.mat
     rng = np.random.default_rng(77)
-    for it in range(400):
+    for it in range(240):
         ql = int(rng.integers(1, 350))
         q = synth.nucl_genome(rng, ql)
         if it % 3 == 0:
@@ -61,9 +59,7 @@ def test_ksw_restatement_vs_reference_random(kso):
             assert np.array_equal(ca, cb), (it, flag)
 
 
-@pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built")
-def test_aligner_restatement_vs_reference_random(kso):
-    ref = Ref()
+def test_aligner_restatement_vs_reference_random(kso, ref):
     rng = np.random.default_rng(78)
     targets = [synth.nucl_genome(rng, int(n)) for n in rng.integers(100, 2000, 20)]
     reads, tasks = synth.nucl_reads(rng, targets, 300, 120, subst=0.06, indel=0.02)

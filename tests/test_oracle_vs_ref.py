@@ -1,17 +1,10 @@
-"""CPU, build container only: oracle/oracle.c against the reference's own sources compiled in place
-(oracle/_ref/libmmseqs_ref.so).  Skipped where /root/reference is absent (the GPU box)."""
+"""CPU: oracle/oracle.c against the reference's own sources (oracle.pyoracle.Ref; the `ref` fixture answers from the recording of
+the reference's outputs in tests/golden)."""
 import numpy as np
 import pytest
 
-from oracle.pyoracle import Ref, pack_targets
+from oracle.pyoracle import pack_targets
 from mmseqs2_b200 import synth
-
-pytestmark = pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built (no /root/reference here)")
-
-
-@pytest.fixture(scope="module")
-def ref():
-    return Ref()
 
 
 def _targets(rng, bg, q, n):
@@ -39,7 +32,7 @@ def test_matrix_fixture_matches_reference(ref, blosum):
 def test_random_pairs_all_entry_points(ref, oracle, blosum, seed):
     rng = np.random.default_rng(seed)
     bg = synth.background(blosum[1])
-    for it in range(8):
+    for it in range(5):
         qL = int(rng.integers(1, 40)) if it % 4 == 0 else int(rng.integers(20, 600))
         q = synth.random_seqs(rng, 1, bg, mean=qL, sigma=0, lo=qL, hi=qL, normal=True)[0]
         if it % 5 == 0:
@@ -53,8 +46,8 @@ def test_random_pairs_all_entry_points(ref, oracle, blosum, seed):
             assert np.array_equal(ref.sw_score_endpos(q, cbf, td, to), oracle.sw_score_endpos(q, cb, bias, td, to))
             a, _, _ = ref.ssw_align(q, cbf, td, to, mode=1)
             assert np.array_equal(a[:, :6], oracle.sw_align(q, cb, bias, td, to))
-        ids = rng.integers(0, len(to) - 1, 2000).astype(np.uint32)
-        dg = rng.integers(-qL - 3, 700, 2000).astype(np.int16).view(np.uint16)
+        ids = rng.integers(0, len(to) - 1, 500).astype(np.uint32)
+        dg = rng.integers(-qL - 3, 700, 500).astype(np.int16).view(np.uint16)
         for use in (True, False):
             cb4 = oracle.round_bias_diag(f) if use else np.zeros(qL, np.int8)
             c1, r1 = ref.diag(q, f if use else None, td, to, ids, dg)
@@ -112,7 +105,7 @@ def test_rescore_diagonal_modes(ref, oracle):
     m = ref.ascii_matrix()
     letters = np.frombuffer(b"ACDEFGHIKLMNPQRSTVWYXBZUacdklmn", np.uint8)
     checked = 0
-    for rep in range(300):
+    for rep in range(60):
         qL, tL = int(rng.integers(1, 400)), int(rng.integers(1, 400))
         q = bytearray(rng.choice(letters, qL).tobytes()); t = bytearray(rng.choice(letters, tL).tobytes())
         if rep % 3 == 0:                                   # a shared segment so that the scores are not all tiny
@@ -128,5 +121,5 @@ def test_rescore_diagonal_modes(ref, oracle):
                 got = oracle.rescore_diagonal(bytes(q), bytes(t), diag, m, mode)
                 assert np.array_equal(got, exp), (rep, diag, mode, got, exp)
                 checked += 1
-    assert checked == 300 * 7 * 5
+    assert checked == 60 * 7 * 5
 

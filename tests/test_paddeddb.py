@@ -61,14 +61,10 @@ def test_writer_layout_properties(gold):
     assert (ty >> 16) & 0x7FFE == 8 and ty & 0xffff == 0
 
 
-def test_writer_on_a_compressed_source(gold, alphabet, tmp_path):
+def test_writer_on_a_compressed_source(gold, alphabet, tmp_path, ref):
     """a source DB written with `createdb --compressed 1` gives the same padded DB (the reader inflates it)"""
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref not built here")
     src = _write_src(gold, tmp_path)
     d, h = db.DB(src), db.DB(src + "_h")
-    ref = Ref()
     csrc = str(tmp_path / "C")
     ref.db_write(csrc, 0, [d.key(i) for i in range(len(d))], [d.data(i) for i in range(len(d))], compressed=True)
     ref.db_write(csrc + "_h", 12, [h.key(i) for i in range(len(h))], [h.data(i) for i in range(len(h))], compressed=True)
@@ -96,16 +92,10 @@ def test_mask_sequence_modes(gold):
                 assert n == int(gold["seq_mask_counts"][k, i]), (k, i)
 
 
-def test_masker_against_live_reference():
-    import ctypes
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref not built here")
-    ref = Ref()
-    lr = np.zeros((21, 21), np.float64)
-    ref.lib.ref_tantan_matrix(lr.ctypes.data_as(ctypes.c_void_p))
+def test_masker_against_live_reference(ref):
+    lr = ref.tantan_matrix()
     rng = np.random.default_rng(5)
-    for t in range(300):
+    for t in range(12):
         L = int(rng.integers(1, 1500))
         if t % 3 == 0:
             s = rng.integers(0, 21, L)
@@ -118,8 +108,7 @@ def test_masker_against_live_reference():
             a = int(rng.integers(0, L))
             s[a:a + 60] = rng.integers(0, 2, len(s[a:a + 60]))
         s = np.ascontiguousarray(s, np.uint8)
-        exp = np.zeros(L, np.float32)
-        ref.lib.ref_tantan_probabilities(s.ctypes.data_as(ctypes.c_void_p), L, exp.ctypes.data_as(ctypes.c_void_p))
+        exp = ref.tantan_probabilities(s)
         assert np.array_equal(db.tantan_probabilities(s, lr).view(np.uint32), exp.view(np.uint32)), t
 
 

@@ -130,7 +130,8 @@ int b200_rescore_diagonal(b200_ctx *ctx, const char *query_data, const uint64_t 
                           const uint32_t *ids, const uint16_t *diagonals, const int8_t *ascii_matrix, int mode, b200_rescore *out);
 
 /* ---- A3-A5: affine-gap local alignment --------------------------------------------------------- */
-/* score only (s_align.score1 as alignScoreEndPos reports it: exact, capped at 32767).  This is the fast path
+/* score only (s_align.score1 as alignScoreEndPos reports it: exact below 32767; a pair whose exact score would pass it reports 32767,
+ * as the reference's saturating word-mode kernel does, and its end and start positions follow that rule too).  This is the fast path
  * (two targets per warp in int16x2); Matcher-level callers run it on every prefilter hit, apply the reference's
  * E-value gate on the host, and ask for positions (below) only for the survivors. */
 int b200_sw_score(b200_ctx *ctx, const b200_query *queries, int n_queries, const b200_pair *pairs, uint64_t n,

@@ -547,6 +547,8 @@ __global__ void pad_profile_kernel(const int8_t *__restrict__ raw, const QueryDe
 // running maximum reaches its final value, end row = smallest row holding it in that column (:233-247, :263-271).
 // DIR=-1 runs the same recurrence on the reversed prefixes query[qEnd..0] x target[dbEnd..0] and stops at the first
 // column whose maximum equals the forward score (alignStartPosBacktrace :1129-1212, `terminate` :259,:435).
+// Word mode adds with adds_epi16, so the diagonal move saturates at 32767 and E and F follow from the saturated H: a pair whose
+// exact score passes 32767 reports 32767 at the first cell that reaches it, and the reverse pass meets 32767 exactly.
 //
 // Lane l owns ROWS consecutive query rows of the current 32*ROWS-row tile and trails lane l-1 by one column; H and F
 // of the boundary row travel by __shfl_up.  Query tiles beyond the first pick their top boundary up from a per-warp
@@ -657,8 +659,8 @@ sw32_kernel(const int8_t *__restrict__ padded, const QueryDesc *__restrict__ qd,
                     for (int j = 0; j < SW_ROWS; j++) {
                         const int s = pp[j];
                         const int e = __viaddmax_s32(E[j], neg_ge, Hg[j]);
-                        int h = __viaddmax_s32_relu(diag, s, e);
-                        h = max(h, f);
+                        // adds_epi16 of the reference's word mode: the diagonal move saturates at 32767 (E and F follow from H)
+                        const int h = __vimax3_s32_relu(__viaddmin_s32(diag, s, 32767), e, f);
                         diag = H[j];
                         H[j] = h;
                         E[j] = e;

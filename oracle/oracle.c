@@ -138,6 +138,7 @@ static int orc_gotoh(const int16_t *mat, int A, const uint8_t *q, const int8_t *
         for (int j = 0; j < qL; j++) {
             int s = mat[(size_t) tr * A + q[(ptrdiff_t) j * qStride]] + cb[(ptrdiff_t) j * qStride];
             int h = diag + s;
+            if (h > 32767) h = 32767;   /* adds_epi16 (word mode) saturates the diagonal move; E and F follow from it */
             int e = E[j + 1];
             if (h < e) h = e;
             if (h < F) h = F;
@@ -174,8 +175,8 @@ void orc_sw_score_endpos(const int16_t *mat, int A, const uint8_t *q, int qL, co
                          const uint8_t *t, int tL, int go, int ge, int32_t *out) {
     int ec, er;
     int max = orc_gotoh(mat, A, q, cb, qL, 1, t, tL, 1, go, ge, -1, &ec, &er);
-    if (max + bias >= 255) {            /* word mode: exact up to INT16_MAX */
-        if (max > 32767) max = 32767;   /* adds_epi16 saturation; unreachable for BASELINE shapes */
+    if (max + bias >= 255) {            /* word mode: every cell saturates at INT16_MAX (orc_gotoh), so a pair whose exact score
+                                           passes 32767 reports 32767 and ends at the first cell that reached it */
         out[0] = max; out[1] = (er < 0) ? qL - 1 : er; out[2] = (ec < 0) ? 0 : ec; out[3] = 1;
     } else if (max == 0) {              /* byte mode, nothing aligned: end_db = -1; pvHmax is all zero so the
                                            trace loop (:263-271) matches index 0 first */

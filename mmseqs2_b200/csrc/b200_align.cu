@@ -2,6 +2,7 @@
 //
 // Kernels (see DESIGN.md for layouts and rooflines):
 //   ungapped_scan_kernel<G,K>  A2  all-diagonals ungapped scan, int16x2 DPX (__viaddmin_s16x2_relu), profile in smem
+//                              (quads of G = 8 queries: half of the profile words from tensor memory, tcgen05.ld)
 //   topk_select_kernel         A2  per-query histogram cut-off + ordered compaction of the u8 score vector
 //   diag_score_kernel          A1  per-(target,diagonal) max-prefix score as a parallel max-subarray reduction
 //   pad_profile_kernel             [A][qlen] int8 -> padded forward / reversed device profiles
@@ -105,8 +106,78 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, unsigned parity) {
 #ifndef B200_SCAN_K3
 #define B200_SCAN_K3 24      // classes up to this K are compiled for B200_SCAN_MINB CTAs per SM
 #endif
-template <int G, int K, bool TILED>
-__global__ void __launch_bounds__(256, TILED ? 1 : (K <= 12 ? 5 : (K <= B200_SCAN_K3 ? B200_SCAN_MINB : 1)))
+
+// Quad variant (QUAD, G = 8 only): a warp scans ONE target for four queries, group q = lane/8 holding query q of the quad.  The
+// residue of a column is then warp-uniform, which is what tcgen05.ld needs: the first R registers of every V-form column come from
+// tensor memory instead of shared memory, halving the shared-memory bytes per cell (the scan's binding resource; DESIGN §3.1).
+// TMEM lane 32*(warp%4) + 8q + g, column a*R + r holds query q's V-form register r of lane g for residue a (each lane quadrant has
+// its own copy).  One 512-thread CTA per SM owns all 512 columns.
+constexpr int kScanQuadThreads = 512;
+constexpr int kScanTmemCols = 512;
+constexpr int kScanQuadMinSmem = 116 * 1024;   // > half of an SM's shared memory: no two quad CTAs (any K) share an SM's TMEM
+__host__ __device__ constexpr int scan_quad_R(int K) { return K <= 22 ? K : 20; }   // 22 residue rows x R <= 512 columns
+
+__device__ __forceinline__ void tmem_fence_sync() {
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+}
+// tcgen05.ld / st of N (16, 8, 4 or 2) consecutive 32-bit columns per lane, shape 32x32b
+template <int N> __device__ __forceinline__ void tmem_ld(uint32_t t, uint32_t *v);
+template <> __device__ __forceinline__ void tmem_ld<16>(uint32_t t, uint32_t *v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
+                   "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+                 : "r"(t));
+}
+template <> __device__ __forceinline__ void tmem_ld<8>(uint32_t t, uint32_t *v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(t));
+}
+template <> __device__ __forceinline__ void tmem_ld<4>(uint32_t t, uint32_t *v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(t));
+}
+template <> __device__ __forceinline__ void tmem_ld<2>(uint32_t t, uint32_t *v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0,%1}, [%2];" : "=r"(v[0]), "=r"(v[1]) : "r"(t));
+}
+template <int N> __device__ __forceinline__ void tmem_st(uint32_t t, const uint32_t *v);
+template <> __device__ __forceinline__ void tmem_st<16>(uint32_t t, const uint32_t *v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(t),
+                 "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
+                 "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]) : "memory");
+}
+template <> __device__ __forceinline__ void tmem_st<8>(uint32_t t, const uint32_t *v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(t), "r"(v[0]), "r"(v[1]), "r"(v[2]),
+                 "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
+}
+template <> __device__ __forceinline__ void tmem_st<4>(uint32_t t, const uint32_t *v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(t), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
+}
+template <> __device__ __forceinline__ void tmem_st<2>(uint32_t t, const uint32_t *v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1,%2};" ::"r"(t), "r"(v[0]), "r"(v[1]) : "memory");
+}
+// R consecutive columns (R even, < 32) as x16 / x8 / x4 / x2 pieces
+template <int R> __device__ __forceinline__ void tmem_ld_cols(uint32_t t, uint32_t *v) {
+    if (R & 16) tmem_ld<16>(t, v);
+    if (R & 8) tmem_ld<8>(t + (R & 16), v + (R & 16));
+    if (R & 4) tmem_ld<4>(t + (R & 24), v + (R & 24));
+    if (R & 2) tmem_ld<2>(t + (R & 28), v + (R & 28));
+}
+template <int R> __device__ __forceinline__ void tmem_st_cols(uint32_t t, const uint32_t *v) {
+    if (R & 16) tmem_st<16>(t, v);
+    if (R & 8) tmem_st<8>(t + (R & 16), v + (R & 16));
+    if (R & 4) tmem_st<4>(t + (R & 24), v + (R & 24));
+    if (R & 2) tmem_st<2>(t + (R & 28), v + (R & 28));
+}
+// wait::ld, then tie the loaded registers to it so that no use of them is scheduled above the wait
+template <int R> __device__ __forceinline__ void tmem_wait_ld(uint32_t *v) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (int i = 0; i < R; i++) asm volatile("" : "+r"(v[i]));
+}
+
+template <int G, int K, bool TILED, bool QUAD>
+__global__ void __launch_bounds__(QUAD ? kScanQuadThreads : 256, QUAD || TILED ? 1 : (K <= 12 ? 5 : (K <= B200_SCAN_K3 ? B200_SCAN_MINB : 1)))
 ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict__ qd, const uint8_t *__restrict__ db,
                      const uint64_t *__restrict__ off, const int32_t *__restrict__ len,
                      const uint32_t *__restrict__ order, uint32_t n_seq, int A, uint8_t *__restrict__ out, uint32_t n_queries,
@@ -114,38 +185,58 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
                      uint32_t *__restrict__ tile_bnd, uint32_t bnd_slot_words) {
     static_assert(K % 2 == 0, "K must be even");
     static_assert(!TILED || G == 32, "the tiled (long-query) variant runs one target per warp");
+    static_assert(!QUAD || (G == 8 && !TILED), "quads are four groups of 8 lanes on one target");
     constexpr int C = K / 4;           // full uint4 chunks of a lane's K registers ...
     constexpr int T = (K % 4) / 2;     // ... plus one uint2 tail chunk when K = 4C + 2
-    // 32-bit words per residue row: [c][g] uint4, then [g] uint2.  With G = 8 a half-warp (the unit of an LDS.64) holds two
-    // groups, i.e. two residue rows: their 64-byte tail chunks would land on the same 16 banks whenever the rows differ by an
-    // even number (r01 ncu: 3-4 % of all wavefronts of <8,22>/<8,26> were such conflicts).  A second copy of the tail 16 words
-    // further on, read by the odd groups, puts the two on disjoint bank halves; the row stride becomes 32(C+1) words, a multiple of 32.
-    constexpr int TAIL2 = (G == 8 && T == 1) ? 16 : 0;
+    // V-form registers [0, R) come from tensor memory (QUAD), the rest from shared memory; R % 4 == 0 whenever R < K
+    constexpr int R = QUAD ? scan_quad_R(K) : 0;
+    constexpr int C_V = R / 4;         // first uint4 chunk of the V table read from shared memory
+    constexpr bool T_V = T && R < K;   // the V tail chunk is read from shared memory
+    // 32-bit words per residue row and query: [c][g] uint4, then [g] uint2.  With G = 8 a half-warp (the unit of an LDS.64) holds
+    // two groups.  Without quads they read two residue rows, and their 64-byte tail chunks would land on the same 16 banks whenever the
+    // rows differ by an even number (r01 ncu: 3-4 % of all wavefronts of <8,22>/<8,26> were such conflicts): a second copy of the tail
+    // 16 words further on, read by the odd groups, puts the two on disjoint bank halves; the row stride becomes 32(C+1) words.
+    // With quads the two groups read one residue row of two queries, ROW_W = 8K = 32C + 16 words apart: disjoint halves already.
+    constexpr int TAIL2 = (G == 8 && T == 1 && !QUAD) ? 16 : 0;
     constexpr int ROW_W = G * K + TAIL2;
+    constexpr int NQ = QUAD ? 4 : 1;   // queries per residue row of the tables, laid out [a][q][c][g]
     extern __shared__ uint4 smem_u4[];
     uint32_t *P = reinterpret_cast<uint32_t *>(smem_u4);
-    uint32_t *Pp = P + (size_t) (A + 1) * ROW_W;
+    uint32_t *Pp = P + (size_t) (A + 1) * NQ * ROW_W;
 
     __shared__ unsigned cur_unit;
+    __shared__ uint32_t tmem_slot;
     const int lane = threadIdx.x & 31;
     const int g = lane % G;
-    constexpr int GROUPS_PER_WARP = 32 / G;
+    constexpr int TARGETS_PER_WARP = QUAD ? 1 : 32 / G;
     const uint32_t warps_per_cta = blockDim.x >> 5;
     const uint32_t warp_in_cta = threadIdx.x >> 5;
     const uint32_t padword = (uint32_t) A * 0x01010101u;
-    const int tail_off = 4 * C * G + (TAIL2 ? ((lane >> 3) & 1) * TAIL2 : 0);   // which copy of the tail chunk this group reads
+    const int q_off = QUAD ? (lane >> 3) * ROW_W : 0;   // this group's query within a residue row of the tables
+    const int tail_off = q_off + 4 * C * G + (TAIL2 ? ((lane >> 3) & 1) * TAIL2 : 0);   // which copy of the tail chunk this group reads
     int cur_q = -1;
     uint32_t cst = 0;
+    uint32_t tmem = 0;                 // QUAD: this warp's lane quadrant of the CTA's 512 columns
+    if (QUAD) {
+        if (warp_in_cta == 0) {
+            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((uint32_t) __cvta_generic_to_shared(&tmem_slot)),
+                         "r"(kScanTmemCols) : "memory");
+            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        }
+        tmem_fence_sync();
+        tmem = tmem_slot + ((uint32_t) (32 * (warp_in_cta & 3)) << 16);
+    }
 
-  // persistent CTA: work units = (query, chunk of the length-sorted target order), handed out query-major / longest
+  // persistent CTA: work units = (query or quad, chunk of the length-sorted target order), handed out query-major / longest
   // targets first by a global counter; the profile tables are rebuilt only when the query changes
   while (true) {
-    __syncthreads();
+    if (QUAD) tmem_fence_sync(); else __syncthreads();
     if (threadIdx.x == 0) cur_unit = atomicAdd(unit_counter, 1u);
     __syncthreads();
     const uint32_t unit = cur_unit;
     if (unit >= n_queries * units_per_query) break;
-    const int qi = (int) (unit / units_per_query);
+    const int qu = (int) (unit / units_per_query);          // query, or quad
+    const int qi = QUAD ? 4 * qu + (lane >> 3) : qu;        // this group's query
     const uint32_t chunk = unit % units_per_query;
     // Query rows are processed in tiles of ROWS = 2*G*K (one tile unless TILED).  Tile p covers rows [p*ROWS, (p+1)*ROWS);
     // in W-form columns it also recomputes row p*ROWS-1 from the boundary words the previous tile left in tile_bnd.
@@ -157,16 +248,15 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
     uint32_t *cta_bnd = TILED ? tile_bnd + (size_t) blockIdx.x * unit_targets * bnd_slot_words : nullptr;
   for (int tile = 0; tile < n_tiles; tile++) {
     const int row_base = tile * ROWS;
-    if (TILED || qi != cur_q) {
+    if (TILED || qu != cur_q) {
         if (TILED) __syncthreads();          // every warp is done with the previous tile's tables (and boundary words)
-        const int8_t *prof = raw + q.raw_off;
-        const int qlen = q.qlen;
-        uint32_t *Pw = P;
-        uint32_t *Ppw = Pp;
         const int words = G * K;
-        for (int idx = threadIdx.x; idx < (A + 1) * words; idx += blockDim.x) {
-            const int a = idx / words, w = idx % words;
+        for (int idx = threadIdx.x; idx < (A + 1) * NQ * words; idx += blockDim.x) {
+            const int a = idx / (NQ * words), qq = idx / words % NQ, w = idx % words;
             const int gg = w / K, r = w % K;
+            const QueryDesc &dq = QUAD ? qd[4 * qu + qq] : q;
+            const int8_t *prof = raw + dq.raw_off;
+            const int qlen = dq.qlen;
             const int r0 = row_base + 2 * w;
             int s0 = 0, s1 = 0, sm1 = 0;  // rows r0, r0+1, r0-1
             if (a < A) {
@@ -175,26 +265,46 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
                 if (r0 + 1 < qlen) s1 = pa[r0 + 1];
                 if (r0 - 1 >= 0 && r0 - 1 < qlen) sm1 = pa[r0 - 1];
             }
-            const int dst = a * ROW_W + (r < 4 * C ? ((r >> 2) * G + gg) * 4 + (r & 3) : 4 * C * G + gg * 2 + (r - 4 * C));
-            Pw[dst] = pack16(s0, s1);
-            Ppw[dst] = pack16(sm1, s0);
-            if (TAIL2 && r >= 4 * C) { Pw[dst + TAIL2] = pack16(s0, s1); Ppw[dst + TAIL2] = pack16(sm1, s0); }
+            const int dst = (a * NQ + qq) * ROW_W + (r < 4 * C ? ((r >> 2) * G + gg) * 4 + (r & 3) : 4 * C * G + gg * 2 + (r - 4 * C));
+            if (r >= R) P[dst] = pack16(s0, s1);
+            Pp[dst] = pack16(sm1, s0);
+            if (TAIL2 && r >= 4 * C) { P[dst + TAIL2] = pack16(s0, s1); Pp[dst + TAIL2] = pack16(sm1, s0); }
+        }
+        if (QUAD && warp_in_cta < 4) {   // one warp per lane quadrant writes that quadrant's copy of V-form registers [0, R)
+            const int8_t *prof = raw + q.raw_off;
+            for (int a = 0; a <= A; a++) {
+                uint32_t v[R > 0 ? R : 1];
+#pragma unroll
+                for (int r = 0; r < R; r++) {
+                    const int r0 = 2 * (g * K + r);
+                    int s0 = 0, s1 = 0;
+                    if (a < A) {
+                        if (r0 < q.qlen) s0 = prof[(size_t) a * q.qlen + r0];
+                        if (r0 + 1 < q.qlen) s1 = prof[(size_t) a * q.qlen + r0 + 1];
+                    }
+                    v[r] = pack16(s0, s1);
+                }
+                tmem_st_cols<R>(tmem + a * R, v);
+            }
+            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         }
         cst = (uint32_t) (255 - q.bias) * 0x00010001u;
-        cur_q = qi;
-        __syncthreads();
+        cur_q = qu;
+        if (QUAD) tmem_fence_sync(); else __syncthreads();
     }
     const bool first_tile = tile == 0, last_tile = tile + 1 == n_tiles;
 
-    for (uint32_t base = chunk * unit_targets + warp_in_cta * GROUPS_PER_WARP; base < unit_end; base += warps_per_cta * GROUPS_PER_WARP) {
-        const uint32_t it = base + lane / G;
+    for (uint32_t base = chunk * unit_targets + warp_in_cta * TARGETS_PER_WARP; base < unit_end; base += warps_per_cta * TARGETS_PER_WARP) {
+        const uint32_t it = base + (QUAD ? 0 : lane / G);
         uint32_t tid = 0;
         int tl = 0;
         if (it < unit_end) { tid = order[it]; tl = len[tid]; }
         const uint4 *tp = reinterpret_cast<const uint4 *>(db + off[tid]);
         int maxl = tl;
+        if (!QUAD) {
 #pragma unroll
-        for (int o = 16; o >= G; o >>= 1) maxl = max(maxl, __shfl_xor_sync(0xffffffffu, maxl, o));
+            for (int o = 16; o >= G; o >>= 1) maxl = max(maxl, __shfl_xor_sync(0xffffffffu, maxl, o));
+        }
 
         uint32_t S[K];
 #pragma unroll
@@ -215,26 +325,37 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
                     bin[0] = b0.x; bin[1] = b0.y; bin[2] = b0.z; bin[3] = b0.w; bin[4] = b1.x; bin[5] = b1.y; bin[6] = b1.z; bin[7] = b1.w;
                 }
             }
+            // QUAD: the V column's tensor-memory words, loaded one column pair ahead (the residue is warp-uniform)
+            uint32_t tv[R > 0 ? R : 1];
+            if (QUAD) tmem_ld_cols<R>(tmem + (cw[0] & 0xffu) * R, tv);
 #pragma unroll
             for (int u = 0; u < 16; u += 2) {
                 // the columns beyond the longest target of the warp are pad residues (neutral row): the second half of the last
                 // 16-column chunk is skipped when nothing real is in it (8-column granularity of the loop end, ~1 % fewer cells)
-                if (!TILED && u == 8 && i0 + 8 >= maxl) break;
+                const bool last_half = !TILED && i0 + 8 >= maxl;
+                if (u == 8 && last_half) break;
                 const uint32_t wv = cw[u >> 2];
                 const uint32_t a0 = (wv >> (8 * (u & 3))) & 0xffu;
                 const uint32_t a1 = (wv >> (8 * ((u + 1) & 3))) & 0xffu;
                 {   // even column: V from W, same registers
-                    const uint32_t *prow = P + a0 * ROW_W;
-                    const uint4 *p = reinterpret_cast<const uint4 *>(prow) + g;
+                    if (QUAD) {
+                        tmem_wait_ld<R>(tv);
 #pragma unroll
-                    for (int c = 0; c < C; c++) {
+                        for (int r = 0; r < R; r++) S[r] = __viaddmin_s16x2_relu(S[r], tv[r], cst);
+                        if (u + 2 < 16 && !(u + 2 == 8 && last_half))
+                            tmem_ld_cols<R>(tmem + ((cw[(u + 2) >> 2] >> (8 * ((u + 2) & 3))) & 0xffu) * R, tv);
+                    }
+                    const uint32_t *prow = P + a0 * NQ * ROW_W;
+                    const uint4 *p = reinterpret_cast<const uint4 *>(prow + q_off) + g;
+#pragma unroll
+                    for (int c = C_V; c < C; c++) {
                         const uint4 x = p[c * G];
                         S[4 * c + 0] = __viaddmin_s16x2_relu(S[4 * c + 0], x.x, cst);
                         S[4 * c + 1] = __viaddmin_s16x2_relu(S[4 * c + 1], x.y, cst);
                         S[4 * c + 2] = __viaddmin_s16x2_relu(S[4 * c + 2], x.z, cst);
                         S[4 * c + 3] = __viaddmin_s16x2_relu(S[4 * c + 3], x.w, cst);
                     }
-                    if (T) {
+                    if (T_V) {
                         const uint2 x = reinterpret_cast<const uint2 *>(prow + tail_off)[g];
                         S[4 * C + 0] = __viaddmin_s16x2_relu(S[4 * C + 0], x.x, cst);
                         S[4 * C + 1] = __viaddmin_s16x2_relu(S[4 * C + 1], x.y, cst);
@@ -246,8 +367,8 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
                 {   // odd column: W from V, shifted by one register
                     uint32_t carry = __shfl_up_sync(0xffffffffu, S[K - 1], 1, G);
                     if (g == 0) carry = TILED ? bin[u >> 1] : 0u;
-                    const uint32_t *prow = Pp + a1 * ROW_W;
-                    const uint4 *p = reinterpret_cast<const uint4 *>(prow) + g;
+                    const uint32_t *prow = Pp + a1 * NQ * ROW_W;
+                    const uint4 *p = reinterpret_cast<const uint4 *>(prow + q_off) + g;
 #ifndef B200_SCAN_NO_PRELOAD
                     uint4 x[C > 0 ? C : 1];
 #pragma unroll
@@ -288,6 +409,10 @@ ungapped_scan_kernel(const int8_t *__restrict__ raw, const QueryDesc *__restrict
         }
     }
   }  // tiles
+  }
+  if (QUAD) {   // every warp's tensor-memory loads have completed (waited) before the columns go back
+      tmem_fence_sync();
+      if (warp_in_cta == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_slot), "r"(kScanTmemCols) : "memory");
   }
 }
 
@@ -1085,17 +1210,22 @@ const ScanCfg kScanCfgs[] = {B200_SCAN_CFGS(B200_SCAN_ENTRY)};
 
 constexpr int kScanCounters = 64;   // one work-unit counter per launch of a batch (launches of one batch may run concurrently)
 
-template <int G, int K, bool TILED>
+// nq counts queries, or quads when QUAD (qd then holds 4 * nq descriptors, quad by quad)
+template <int G, int K, bool TILED, bool QUAD>
 cudaError_t launch_scan_cfg(b200_ctx *ctx, const int8_t *raw, const QueryDesc *qd, int nq, uint8_t *dense, cudaStream_t stream, int counter_slot) {
-    const size_t smem = (size_t) 2 * (ctx->alphabet + 1) * (K * G + ((G == 8 && K % 4 == 2) ? 16 : 0)) * sizeof(uint32_t);
-    cudaError_t e = cudaFuncSetAttribute(ungapped_scan_kernel<G, K, TILED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+    const int threads = QUAD ? kScanQuadThreads : 256;
+    size_t smem = (size_t) 2 * (ctx->alphabet + 1) * (QUAD ? 4 : 1) * (K * G + ((G == 8 && K % 4 == 2 && !QUAD) ? 16 : 0)) * sizeof(uint32_t);
+    if (QUAD) smem = std::max<size_t>(smem, kScanQuadMinSmem);
+    cudaError_t e = cudaFuncSetAttribute(ungapped_scan_kernel<G, K, TILED, QUAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
     if (e != cudaSuccess) return e;
     int per_sm = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ungapped_scan_kernel<G, K, TILED>, 256, smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ungapped_scan_kernel<G, K, TILED, QUAD>, threads, smem);
     if (e != cudaSuccess) return e;
+    // a quad CTA allocates all of an SM's tensor memory: a second one on the SM would block in tcgen05.alloc
+    if (QUAD && per_sm != 1) return cudaErrorInvalidConfiguration;
     per_sm = std::max(per_sm, 1);
     const uint64_t resident = (uint64_t) ctx->sm_count * per_sm;
-    const uint32_t groups_per_cta = 256 / G;
+    const uint32_t groups_per_cta = QUAD ? threads / 32 : 256 / G;   // targets per CTA-wide pass
     // ~16 work units per resident CTA over the whole launch, each a multiple of one CTA-wide pass over the sorted targets
     uint64_t unit_targets = ((uint64_t) ctx->n_seq * nq + resident * 16 - 1) / (resident * 16);
     unit_targets = std::max<uint64_t>(groups_per_cta, (unit_targets + groups_per_cta - 1) / groups_per_cta * groups_per_cta);
@@ -1111,22 +1241,34 @@ cudaError_t launch_scan_cfg(b200_ctx *ctx, const int8_t *raw, const QueryDesc *q
         e = ctx->bnd.reserve(sizeof(uint32_t) * (size_t) slot_words * unit_targets * ctas);
     }
     if (e != cudaSuccess) return e;
-    ungapped_scan_kernel<G, K, TILED><<<(unsigned) ctas, 256, smem, stream>>>(
+    ungapped_scan_kernel<G, K, TILED, QUAD><<<(unsigned) ctas, threads, smem, stream>>>(
         raw, qd, ctx->d_res, ctx->d_off, ctx->d_len, ctx->d_order, (uint32_t) ctx->n_seq, ctx->alphabet, dense, (uint32_t) nq, units_per_query,
         (uint32_t) unit_targets, counter, TILED ? ctx->bnd.as<uint32_t>() : nullptr, slot_words);
     ctx->launches++;
     return cudaGetLastError();
 }
 
-// queries of one launch must share a (G,K) configuration; the caller groups them by capacity class
-cudaError_t launch_scan(b200_ctx *ctx, int cfg, const int8_t *raw, const QueryDesc *qd, int nq, uint8_t *dense, cudaStream_t stream, int counter_slot) {
+template <int G, int K>
+cudaError_t launch_scan_quads(b200_ctx *ctx, const int8_t *raw, const QueryDesc *qd, int nq, uint8_t *dense, cudaStream_t stream, int counter_slot) {
+    if constexpr (G == 8) return launch_scan_cfg<8, K, false, true>(ctx, raw, qd, nq, dense, stream, counter_slot);
+    return cudaErrorInvalidValue;
+}
+
+// queries of one launch must share a (G,K) configuration; the caller groups them by capacity class (quad: nq quads of 4 queries)
+cudaError_t launch_scan(b200_ctx *ctx, int cfg, bool quad, const int8_t *raw, const QueryDesc *qd, int nq, uint8_t *dense, cudaStream_t stream,
+                        int counter_slot) {
     switch (cfg) {
-#define B200_SCAN_CASE(n, g, k) case n: return launch_scan_cfg<g, k, false>(ctx, raw, qd, nq, dense, stream, counter_slot);
+#define B200_SCAN_CASE(n, g, k) \
+    case n: return quad ? launch_scan_quads<g, k>(ctx, raw, qd, nq, dense, stream, counter_slot) \
+                        : launch_scan_cfg<g, k, false, false>(ctx, raw, qd, nq, dense, stream, counter_slot);
         B200_SCAN_CFGS(B200_SCAN_CASE)
 #undef B200_SCAN_CASE
-        default: return launch_scan_cfg<32, 32, true>(ctx, raw, qd, nq, dense, stream, counter_slot);   // queries longer than 2047: row tiles of 2048
+        default: return launch_scan_cfg<32, 32, true, false>(ctx, raw, qd, nq, dense, stream, counter_slot);   // queries longer than 2047: row tiles of 2048
     }
 }
+
+// quads need the R tensor-memory columns of every residue row (pad row included) to fit the SM's 512; R is largest at K = 22
+bool scan_quads_fit(int alphabet) { return (alphabet + 1) * scan_quad_R(22) <= kScanTmemCols; }
 
 int scan_cfg_for(int qlen) {
     const int n = (int) (sizeof(kScanCfgs) / sizeof(kScanCfgs[0]));
@@ -1189,8 +1331,8 @@ struct b200_job {
     // scan
     int nq = 0, thr = 0;
     uint32_t k = 0;
-    std::vector<int> cfg_of_query;             // per query
-    std::vector<std::vector<int>> cfg_groups;  // query indices per configuration (launch groups)
+    struct ScanGroup { int cfg; bool quad; std::vector<int> queries; };   // one configuration's launch; quad: 4 queries per quad
+    std::vector<ScanGroup> scan_groups;
     DevBuf raw, qdesc, qdesc_grouped, dense, hits, nhits, pad, part_hist;
     std::vector<int> grouped_order;  // position -> original query index
     // sw
@@ -1454,11 +1596,31 @@ int b200_scan_job_create(b200_ctx *ctx, const b200_query *queries, int nq, int m
     }
     b200_job *job = new b200_job();
     job->ctx = ctx; job->kind = 1; job->nq = nq; job->thr = min_score_excl; job->k = max_hits;
-    job->cfg_groups = groups;
+    // The G = 8 queries go four to a launch unit (quads, see ungapped_scan_kernel): sorted by length, longest first, each quad in
+    // the class of its longest query.  The n mod 4 shortest stay in their own classes, as do G = 16/32 and tiled queries.
+    // B200_SCAN_NO_QUADS=1 turns quads off (A/B measurements).
+    std::vector<std::vector<int>> quad_groups(groups.size());
+    if (getenv("B200_SCAN_NO_QUADS") == nullptr && scan_quads_fit(A)) {
+        std::vector<int> g8;
+        for (size_t c = 0; c < groups.size(); c++)
+            if (c < sizeof(kScanCfgs) / sizeof(kScanCfgs[0]) && kScanCfgs[c].G == 8) { g8.insert(g8.end(), groups[c].begin(), groups[c].end()); groups[c].clear(); }
+        std::stable_sort(g8.begin(), g8.end(), [queries](int a, int b) { return queries[a].qlen > queries[b].qlen; });
+        const size_t n_quad = g8.size() / 4 * 4;
+        for (size_t i = 0; i < n_quad; i += 4) {
+            std::vector<int> &qg = quad_groups[scan_cfg_for(queries[g8[i]].qlen)];
+            qg.insert(qg.end(), g8.begin() + i, g8.begin() + i + 4);
+        }
+        for (size_t i = n_quad; i < g8.size(); i++) groups[scan_cfg_for(queries[g8[i]].qlen)].push_back(g8[i]);
+        for (auto &gr : groups) std::sort(gr.begin(), gr.end());
+    }
+    for (size_t c = 0; c < groups.size(); c++) {
+        if (!quad_groups[c].empty()) job->scan_groups.push_back({(int) c, true, quad_groups[c]});
+        if (!groups[c].empty()) job->scan_groups.push_back({(int) c, false, groups[c]});
+    }
     std::vector<QueryDesc> h_qd;
     uint64_t raw_bytes = 0;
-    for (size_t c = 0; c < groups.size(); c++)
-        for (int qi : groups[c]) {
+    for (const auto &sg : job->scan_groups)
+        for (int qi : sg.queries) {
             QueryDesc d;
             memset(&d, 0, sizeof(d));
             d.qlen = queries[qi].qlen; d.bias = queries[qi].bias; d.raw_off = raw_bytes;
@@ -1494,17 +1656,17 @@ int b200_scan_job_create(b200_ctx *ctx, const b200_query *queries, int nq, int m
 // one boundary scratch and stays on the ctx stream.
 static int scan_job_run_locked(b200_job *job) {
     b200_ctx *ctx = job->ctx;
-    struct L { int cfg, pos, n; };
+    struct L { int cfg; bool quad; int pos, n; };   // n queries, or n quads
     std::vector<L> launches;
     int pos = 0;
-    for (size_t c = 0; c < job->cfg_groups.size(); c++) {
-        const int n = (int) job->cfg_groups[c].size();
-        // grid.y is limited to 65535
-        for (int s = 0; s < n; s += 32768) launches.push_back({(int) c, pos + s, std::min(32768, n - s)});
-        pos += n;
+    for (const auto &sg : job->scan_groups) {
+        const int per = sg.quad ? 4 : 1;
+        const int n = (int) sg.queries.size() / per;
+        for (int s = 0; s < n; s += 32768) launches.push_back({sg.cfg, sg.quad, pos + per * s, std::min(32768, n - s)});
+        pos += (int) sg.queries.size();
     }
     const int n_cfg = (int) (sizeof(kScanCfgs) / sizeof(kScanCfgs[0]));
-    auto weight = [n_cfg](const L &l) { return (double) l.n * (l.cfg < n_cfg ? 2.0 * kScanCfgs[l.cfg].G * kScanCfgs[l.cfg].K : 1e9); };
+    auto weight = [n_cfg](const L &l) { return (double) l.n * (l.quad ? 4 : 1) * (l.cfg < n_cfg ? 2.0 * kScanCfgs[l.cfg].G * kScanCfgs[l.cfg].K : 1e9); };
     std::stable_sort(launches.begin(), launches.end(), [&weight](const L &a, const L &b) { return weight(a) > weight(b); });
     const bool fan_out = launches.size() > 1 && getenv("B200_SCAN_SERIAL") == nullptr;
     if (fan_out) CU_TRY(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -1518,7 +1680,7 @@ static int scan_job_run_locked(b200_job *job) {
             st = ctx->side[k];
             if (!used[k]) { CU_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_fork, 0)); used[k] = true; }
         }
-        CU_TRY(ctx, launch_scan(ctx, l.cfg, job->raw.as<int8_t>(), job->qdesc.as<QueryDesc>() + l.pos, l.n,
+        CU_TRY(ctx, launch_scan(ctx, l.cfg, l.quad, job->raw.as<int8_t>(), job->qdesc.as<QueryDesc>() + l.pos, l.n,
                                 job->dense.as<uint8_t>() + (size_t) l.pos * ctx->n_seq, st, (int) (i % kScanCounters)));
     }
     for (int k = 0; k < 3; k++)
